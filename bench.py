@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- decode Mpixels/s of the VarDCT transform pipeline on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (dequant+CfL+LLF+IDCT -> Gaborish -> EPF -> XYB->linear RGB)
 over one frame of synthetic content.
@@ -193,6 +193,19 @@ def host_cpu_info() -> dict:
             continue
     eff = aff if quota is None else max(1, min(aff, int(math.ceil(quota))))
     return {"cores": eff, "affinity": aff, "cgroup_quota": quota, "os_cpu_count": total}
+
+
+DUMP_BYTES = 60_000_000   # --dump-outputs: what one run writes stays under 64 MB with the .npy headers
+
+
+def output_sample(kind: str, frame: np.ndarray, budget: int) -> dict[str, np.ndarray]:
+    """What --dump-outputs writes for one output kind: the whole frame as float32 when it fits in `budget`
+    bytes, otherwise a fixed sample (seed 0, so two runs of the same workload pick the same samples) with its
+    flat indices as float64 (exact below 2**53)."""
+    if frame.size * 4 <= budget:
+        return {kind: frame.astype(np.float32)}
+    idx = np.unique(np.random.default_rng(0).integers(0, frame.size, budget // 12))
+    return {kind: frame.reshape(-1)[idx].astype(np.float32), f"{kind}_index": idx.astype(np.float64)}
 
 
 def geomean_excluding_first(secs, px: int) -> float:
@@ -493,7 +506,13 @@ def main() -> int:
                          "chunks stored to all peers by a copy kernel; p2p: peer stores fused into the filter kernel; multicast: "
                          "multimem.st through the NVSwitch; nccl: all_gather_into_tensor after the kernels; auto (default) = ce, "
                          "except sm for the f32 frame on 4 and more GPUs (DESIGN.md section 6)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frame of the last device-resident step of every measured "
+                         "output kind to DIR/<kind>.npy as float32 (a seeded sample of at most 64 MB in all, with its "
+                         "flat indices in DIR/<kind>_index.npy, when the whole frame does not fit)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "64x1080p"):
+        ap.error("--dump-outputs is supported for the single-frame b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.gather in ("p2p", "multicast"):
         os.environ["JXLGPU_GATHER"] = "kernel"   # (read when the context is created)
@@ -625,6 +644,13 @@ def main() -> int:
                 gather_mode = "NCCL all_gather_into_tensor after the filter kernel"
             my_out = gathered[rank]
 
+        def whole_frame() -> np.ndarray:
+            """The frame as rank 0 holds it: every band, as it arrived in its frame buffer."""
+            if world == 1:
+                return gathered.cpu().numpy()
+            return np.concatenate([gathered[r, :sharding.band_pixel_rows(desc, *bands[r])[1]].cpu().numpy()
+                                   for r in range(world)])
+
         def step():
             pipe.render_device(my_out.data_ptr(), row_bytes, stream.cuda_stream)
             if world > 1:
@@ -649,6 +675,8 @@ def main() -> int:
         ev1.record(stream)
         torch.cuda.synchronize()
         barrier()
+        if args.dump_outputs and rank == 0:
+            dumps.update(output_sample(kind, whole_frame(), DUMP_BYTES // len(kinds)))
         ms_total = ev0.elapsed_time(ev1)
         launches = pipe.launch_count() - launches0
         clocks = None   # the sampler keeps running through this output kind's e2e arm (see the end of measure)
@@ -678,11 +706,7 @@ def main() -> int:
         if fr.get("decoded") is None and rank == 0 and full and kind == "f32":
             # no cached pixels of the reference decoder: compare with the reference's own hot path (big frames)
             # or, for synthetic coefficient frames, with the C oracle on the first 512 rows
-            if world == 1:
-                got = gathered.cpu().numpy()
-            else:
-                got = np.concatenate([gathered[r, :sharding.band_pixel_rows(desc, *bands[r])[1]].cpu().numpy()
-                                      for r in range(world)])
+            got = whole_frame()
             from oracle import ref
             if fr.get("jxl") is not None and ref.available():
                 frame = ref.Frame(fr["jxl"], host_cpu_info()["cores"])
@@ -709,11 +733,7 @@ def main() -> int:
                 parity = {"bit_exact_vs_oracle": bool(np.array_equal(got[:rows - halo], want[:rows - halo])),
                           "rows_checked": int(rows - halo)}
         if fr.get("decoded") is not None and rank == 0 and full:
-            if world == 1:
-                got = gathered.cpu().numpy()
-            else:  # every band, as it arrived in rank 0's frame buffer
-                got = np.concatenate([gathered[r, :sharding.band_pixel_rows(desc, *bands[r])[1]].cpu().numpy()
-                                      for r in range(world)])
+            got = whole_frame()
             if kind == "f32":
                 want = fr["decoded"][:got.shape[0]]
                 d = np.abs(got - want)
@@ -836,10 +856,16 @@ def main() -> int:
         return res
 
     shared = {}
+    dumps = {}
+    other_kind = "srgb8" if args.output == "f32" else "f32"
+    kinds = [args.output] if args.no_variants else [args.output, other_kind]
     pipeline.pin_side_info(desc)   # side info in page-locked memory, as the coefficient blocks are
     primary = measure(args.output, True)
-    other_kind = "srgb8" if args.output == "f32" else "f32"
     variant = None if args.no_variants else measure(other_kind, True)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name_, a in dumps.items():
+            np.save(os.path.join(args.dump_outputs, f"{name_}.npy"), a)
     desc.out_format = abi.OUT_RGB_F32 if args.output == "f32" else abi.OUT_RGB_U8
     value, ms_step, launches, clocks = primary["value"], primary["ms_per_step"], primary["launches"], primary["clocks"]
     kavg, parity, gather_mode = primary["kernel_ms"], primary["parity"], primary["gather_mode"]

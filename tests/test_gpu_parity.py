@@ -350,22 +350,22 @@ def test_upsampling_bit_exact(pipe, n, w, h, fmt, srgb):
 
 @pytest.mark.parametrize("rs", [2, 4, 8])
 def test_upsampled_reference_frames(pipe, rs):
-    """Codestreams the reference encoder made with resampling 2 / 4 / 8 (tests/golden/upsampling_weights.npz):
-    entropy-decoded by the reference, rendered here, compared with the reference decoder's own pixels."""
-    from pathlib import Path
-    from oracle import cpu, ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    data = bytes(np.load(Path(__file__).parent / "golden" / "upsampling_weights.npz")[f"jxl{rs}"])
-    fr = ref.Frame(data, 2)
-    d = fr.dump()
-    fr.close()
+    """Frames the reference encoder made with resampling 2 / 4 / 8, entropy-decoded by the reference, rendered here,
+    compared with the reference decoder's own pixels (tests/golden/vs_reference.npz.xz: the hand-off and the digest of
+    the pixels of its -ffp-contract=off build, which the restatement in host-rcpss mode reproduces bit for bit)."""
+    from oracle import cpu
+    z = support.load_xz_npz(support.GOLDEN / "vs_reference.npz.xz")
+    support.require_host_rcpss(z)
+    d = support.load_dump(z, f"ups{rs}")
     desc = cpu.desc_from_dump(d)
     assert desc.upsampling == rs
     got = pipe.decode_frame(desc, d.coeffs)
-    assert got.shape == d.decoded.shape
+    assert got.shape == (d.info.ysize_upsampled, d.info.xsize_upsampled, 3)
     assert_same(got, oracle(desc, d.coeffs), f"resampling {rs} vs oracle")
-    assert np.abs(got - d.decoded).max() <= 2e-5       # vs the reference decoder (rcpps in AdjustQuantBias)
+    desc.out_format = abi.OUT_PLANAR_F32
+    want = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
+    assert support.digest(want) == z[f"ups{rs}.want"][0].tobytes()
+    assert np.abs(got - np.moveaxis(want, 0, 2)).max() <= 2e-5       # vs the reference decoder (rcpps in AdjustQuantBias)
 
 
 @pytest.mark.parametrize("n,w,h", [(1, 1201, 531), (2, 600, 270)])
@@ -430,20 +430,19 @@ def test_ycbcr_colour_transform_bit_exact(pipe, fmt):
 
 def test_jpeg_origin_frame_against_the_reference_decoder(pipe):
     """A 4:4:4 JPEG, recompressed by the reference encoder, entropy-decoded by the reference, rendered here: the 8-bit
-    pixels are the reference decoder's."""
-    pytest.importorskip("PIL")
-    from oracle import cpu, ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    from tests.test_oracle_vs_reference import make_jpeg
-    data = ref.encode_jpeg(make_jpeg(1000, 700, 85), 4)
-    fr = ref.Frame(data, 2)
-    d = fr.dump()
-    fr.close()
+    pixels are the reference decoder's (tests/golden/vs_reference.npz.xz: the hand-off and the digest of the public
+    decoder's pixels, which the restatement in host-rcpss mode reproduces bit for bit)."""
+    from oracle import cpu
+    from tests.test_oracle_vs_reference import JPEG_CASES
+    w, h, q = JPEG_CASES[0]
+    z = support.load_xz_npz(support.GOLDEN / "vs_reference.npz.xz")
+    support.require_host_rcpss(z)
+    d = support.load_dump(z, f"jpeg{w}x{h}_{q}")
     desc = cpu.desc_from_dump(d)
     assert desc.color_transform == 1
     desc.out_format = abi.OUT_RGB_U8
+    want = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
+    assert support.digest(want) == z[f"jpeg{w}x{h}_{q}.want"][1].tobytes()
     got = pipe.decode_frame(desc, d.coeffs)
-    want = ref.decode_native(data, (700, 1000, 3), np.uint8, 2)
     diff = np.abs(got.astype(np.int16) - want.astype(np.int16))
     assert diff.max() <= 1 and (diff != 0).mean() < 1e-3      # (rcpps in AdjustQuantBias may cross a rounding boundary)

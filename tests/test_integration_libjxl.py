@@ -18,9 +18,10 @@ import numpy as np
 import pytest
 
 import jxl_workload as wl
+from oracle import build_ref
 
 ROOT = Path(__file__).resolve().parents[1]
-REF_ROOT = Path(os.environ.get("JXL_REFERENCE_ROOT", "/root/reference"))
+HAVE_REF_TREE = build_ref.reference_present()
 
 # peak error of linear RGB in [0,1] against the stock CPU decoder (ISO 18181-3 tooling default is 1e-3,
 # tools/conformance/tooling_test.sh:49-50; the reference's fast-vs-simple pipeline bound is 2e-4)
@@ -30,10 +31,10 @@ TOL_PEAK = 2e-5
 def need_gpu_variant():
     from oracle import ref
     if not ref.available("gpu"):
-        if REF_ROOT.exists():
+        if HAVE_REF_TREE:
             pytest.fail("oracle/_ref/libjxl_ref_harness_gpu.so missing although the reference is present: "
                         "run `python oracle/build_ref.py` (after building libjxl_b200.so)")
-        pytest.skip("integrated reference variant not built (no /root/reference on this box)")
+        pytest.skip("integrated reference variant not built (no reference source tree)")
     return ref
 
 
@@ -87,9 +88,9 @@ def run_child(mode, cases, sparse=True):
 
 def test_patch_anchors_match_the_reference(tmp_path):
     """integration/patch_libjxl.py applies cleanly (every anchor exactly once) to the reference as it is."""
-    if not REF_ROOT.exists():
-        pytest.skip("no reference tree on this box")
-    subprocess.check_call([sys.executable, str(ROOT / "integration" / "patch_libjxl.py"), str(REF_ROOT), str(tmp_path)])
+    if not HAVE_REF_TREE:
+        pytest.skip("no reference source tree")
+    subprocess.check_call([sys.executable, str(ROOT / "integration" / "patch_libjxl.py"), str(build_ref.REF), str(tmp_path)])
     for name in ("dec_frame.cc", "dec_group.cc"):
         assert "jxlb_integration::" in (tmp_path / "lib" / "jxl" / name).read_text()
 

@@ -119,7 +119,7 @@ def test_packed_outputs_against_reference(case):
     the reference's own FromLinear/WriteToOutput stages.  Exact-reciprocal mode, so the 12-bit rcpps of
     the reference's AdjustQuantBias may move a value across a rounding boundary: at most one code
     value, on a small fraction of the samples (f32: absolute 2e-5).  tests/test_oracle_vs_reference.py
-    holds the bit-exact version of this comparison (host-rcpss mode, needs oracle/_ref)."""
+    holds the bit-exact version of this comparison (host-rcpss mode)."""
     from oracle import cpu
     fmt, mask = OUTPUT_CASES[case]
     desc, coeffs, _ = support.golden_desc(out_format=fmt, stage_mask=mask)

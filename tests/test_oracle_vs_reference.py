@@ -1,6 +1,7 @@
-"""Pins oracle/jxl_oracle.c against the UNMODIFIED reference compiled here by
-oracle/build_ref.py (skipped where oracle/_ref is absent, e.g. a box without /root/reference
-and without the prebuilt .so).  strict build = -ffp-contract=off => bit-exact expected."""
+"""Pins oracle/jxl_oracle.c against the UNMODIFIED reference.  The reference's outputs (strict build =
+-ffp-contract=off, so bit-exact is expected) and the coefficient hand-offs of the frames it encoded are stored
+in tests/golden/vs_reference.npz.xz (tests/golden/make_vs_reference.py); the tests that drive the reference's own
+decoder through the integration headers need oracle/_ref, compiled by oracle/build_ref.py, and skip without it."""
 import numpy as np
 import pytest
 
@@ -10,15 +11,61 @@ from tests import support
 
 pytestmark = pytest.mark.usefixtures("built")
 
+# The golden data stores every frame's coefficients, so the frames are small; each still spans more than one
+# 256x256 group (the reference's decoder does not hand single-group frames to the hot path).
+STAGE_FRAMES = [
+    dict(w=261, h=85, distance=1.0, gaborish=1, epf=3, kind="photo"),      # odd size, full chain
+    dict(w=264, h=96, distance=1.0, gaborish=-1, epf=-1, kind="photo"),    # BASELINE config 1 settings (defaults: gab, epf 1)
+    dict(w=264, h=48, distance=0.5, gaborish=0, epf=0, kind="photo"),      # no filters: dequant+IDCT+XYB only
+    dict(w=264, h=136, distance=3.0, gaborish=1, epf=2, kind="smooth"),    # large transforms (up to 64x64)
+]
+OUTPUT_FRAME = (259, 61)
+OUTPUT_STAGE_CASES = [(abi.OUT_RGB_F32, True), (abi.OUT_RGB_U8, True), (abi.OUT_RGBA_U8, True), (abi.OUT_RGB_U16, True),
+                      (abi.OUT_RGB_F16, True), (abi.OUT_RGB_U8, False), (abi.OUT_RGB_F16, False)]
+PUBLIC_CASES = [(abi.OUT_RGB_U8, np.uint8, 3), (abi.OUT_RGBA_U8, np.uint8, 4), (abi.OUT_RGB_U16, np.uint16, 3),
+                (abi.OUT_RGB_F16, np.float16, 3), (abi.OUT_RGB_F32, np.float32, 3)]
+DC_CASES = [(256, 256), (960, 540), (37, 21)]
+UPSAMPLING_CASES = [(2, 600, 300), (4, 1100, 210), (8, 2100, 160)]
+NOISE_CASES = [(1, 300, 150, 3200), (2, 600, 299, 6400), (1, 261, 130, 1600)]
+JPEG_CASES = [(300, 150, 90), (261, 165, 75)]
+
+
+@pytest.fixture(scope="module")
+def golden():
+    return support.load_xz_npz(support.GOLDEN / "vs_reference.npz.xz")
+
+
+@pytest.fixture(scope="module")
+def host_rcpss(golden):
+    support.require_host_rcpss(golden)
+
+
+def chain(info) -> int:
+    return (1 if info.gab else 0) | (2 if info.epf_iters >= 3 else 0) | (4 if info.epf_iters >= 1 else 0) | \
+        (8 if info.epf_iters >= 2 else 0)
+
+
+def stage_masks(info) -> list[int]:
+    """Every stage prefix of the frame's chain (and the chain with XYB) that test_frames_stage_by_stage renders."""
+    frame_mask = chain(info)
+    masks = [0, 16, frame_mask, frame_mask | 16]
+    if info.epf_iters > 0:
+        masks += [1, 1 | 4, 2 | 4 | 8]
+    return masks
+
+
+def same(got: np.ndarray, want_digest: np.ndarray) -> bool:
+    return support.digest(got) == want_digest.tobytes()
+
 
 @pytest.fixture(scope="module")
 def refmod(ref_available):
+    from oracle import build_ref
     if not ref_available:
-        import os
-        if os.path.isdir(os.environ.get("JXL_REFERENCE_ROOT", "/root/reference")):
+        if build_ref.reference_present():
             pytest.fail("oracle/_ref is not built although the reference is present: the oracle (and the tables it "
                         "shares with the product, csrc/jxl_tables.h) would go unpinned -- run `python oracle/build_ref.py`")
-        pytest.skip("oracle/_ref not built (no reference on this box)")
+        pytest.skip("oracle/_ref not built (no reference source tree)")
     from oracle import ref
     ref.use_variant("strict")
     yield ref
@@ -26,57 +73,41 @@ def refmod(ref_available):
 
 
 @pytest.mark.parametrize("strategy", range(27))
-def test_all_strategies_bit_exact(strategy, refmod):
+def test_all_strategies_bit_exact(strategy, golden):
     from oracle import cpu
     rng = np.random.default_rng(1000 + strategy)
     r, c = abi.COVERED_Y[strategy] * 8, abi.COVERED_X[strategy] * 8
+    want = golden[f"strategy{strategy}"]
     for trial in range(2):
         co = (rng.laplace(0, 1.0, r * c) * (rng.random(r * c) < 0.3)).astype(np.float32)
-        assert np.array_equal(refmod.transform_to_pixels(strategy, co, r, c), cpu.transform_to_pixels(strategy, co))
+        assert same(cpu.transform_to_pixels(strategy, co), want[trial]), trial
     dc = rng.normal(0, 1, (abi.COVERED_Y[strategy], abi.COVERED_X[strategy])).astype(np.float32)
-    z = np.zeros(r * c, np.float32)
-    assert np.array_equal(refmod.llf_from_dc(strategy, dc, z), cpu.llf_from_dc(strategy, dc, z))
+    assert same(cpu.llf_from_dc(strategy, dc, np.zeros(r * c, np.float32)), want[2])
 
 
-@pytest.mark.parametrize("cfg", [
-    dict(w=517, h=331, distance=1.0, gaborish=1, epf=3),      # odd size, full chain
-    dict(w=512, h=512, distance=1.0, gaborish=-1, epf=-1),    # BASELINE config 1 (defaults: gab, epf 1)
-    dict(w=300, h=520, distance=0.5, gaborish=0, epf=0),      # no filters: dequant+IDCT+XYB only
-    dict(w=640, h=264, distance=3.0, gaborish=1, epf=2, kind="smooth"),  # large transforms
-])
-def test_frames_stage_by_stage(cfg, refmod):
+@pytest.mark.parametrize("cfg", range(len(STAGE_FRAMES)), ids=[f"cfg{k}" for k in range(len(STAGE_FRAMES))])
+def test_frames_stage_by_stage(cfg, golden, host_rcpss):
     """Every stage prefix, hot path only, same coefficients: the reference's own
     DecodeGroupForRoundtrip + stages vs the C restatement. rcp_mode 1 (host rcpss, what the
-    reference's AVX2 path executes on this machine) must be bit-exact; rcp_mode 0 (exact
-    reciprocal = what the CUDA path computes) within 2e-5 absolute."""
+    reference's AVX2 path executes) must be bit-exact; rcp_mode 0 (exact reciprocal = what the
+    CUDA path computes) within 2e-5 absolute."""
     from oracle import cpu
-    kind = cfg.pop("kind", "photo")
-    img = wl.synth_image(cfg["w"], cfg["h"], 77, kind)
-    data = refmod.encode_rgb8(img, cfg["distance"], 7, cfg["gaborish"], cfg["epf"], 2)
-    fr = refmod.Frame(data, 2)
-    d = fr.dump()
+    d = support.load_dump(golden, f"stage{cfg}")
     desc = cpu.desc_from_dump(d, out_format=abi.OUT_PLANAR_F32)
-    frame_mask = (1 if d.info.gab else 0) | (2 if d.info.epf_iters >= 3 else 0) | \
-        (4 if d.info.epf_iters >= 1 else 0) | (8 if d.info.epf_iters >= 2 else 0)
-    masks = [0, 16, frame_mask, frame_mask | 16]
-    if d.info.epf_iters > 0:
-        masks += [1, 1 | 4, 2 | 4 | 8]
-    for mask in sorted(set(masks)):
-        want, _ = fr.render(mask)
+    masks = golden[f"stage{cfg}.masks"].tolist()
+    assert masks == sorted(set(stage_masks(d.info)))
+    for mask, want in zip(masks, golden[f"stage{cfg}.want"]):
         desc.stage_mask = abi.STAGE_EXPLICIT | mask
         got1 = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
-        assert np.array_equal(got1, want), (mask, float(np.abs(got1 - want).max()))
+        assert same(got1, want), mask
         got0 = cpu.render_frame(desc, d.coeffs, rcp_mode=0)
-        assert np.abs(got0 - want).max() <= 2e-5, mask
+        assert np.abs(got0 - got1).max() <= 2e-5, mask
     # and the full public-API decode of the default-flag build (compiler-made FMAs differ)
-    refmod.use_variant("default")
-    full = refmod.decode_linear_f32(data, 1)
-    refmod.use_variant("strict")
     desc.stage_mask = 0
     desc.out_format = abi.OUT_RGB_F32
     got = cpu.render_frame(desc, d.coeffs, rcp_mode=0)
-    assert np.abs(got - full).max() <= 5e-5
-    fr.close()
+    full = golden[f"stage{cfg}.full_sample"]
+    assert np.abs(got.reshape(-1)[support.sample_index(got.size)] - full).max() <= 5e-5
 
 
 def test_hot_path_render_equals_public_decode(refmod):
@@ -96,69 +127,47 @@ def test_hot_path_render_equals_public_decode(refmod):
         refmod.use_variant("strict")
 
 
-@pytest.mark.parametrize("fmt,srgb", [(abi.OUT_RGB_F32, True), (abi.OUT_RGB_U8, True), (abi.OUT_RGBA_U8, True),
-                                      (abi.OUT_RGB_U16, True), (abi.OUT_RGB_F16, True), (abi.OUT_RGB_U8, False),
-                                      (abi.OUT_RGB_F16, False)])
-def test_output_stages_bit_exact(fmt, srgb, refmod):
+@pytest.mark.parametrize("fmt,srgb", OUTPUT_STAGE_CASES)
+def test_output_stages_bit_exact(fmt, srgb, golden, host_rcpss):
     """FromLinearStage<OpRgb> + WriteToOutputStage (dithered u8, RGBA, u16, binary16, f32) of the strict
     reference build vs the restatement, whole frame, host-rcpss mode: identical bytes."""
     from oracle import cpu
-    img = wl.synth_image(333, 277, 5)
-    data = refmod.encode_rgb8(img, 1.0, 7, -1, 2, 2)
-    fr = refmod.Frame(data, 2)
-    d = fr.dump()
-    want, _ = fr.render_out(-33 if srgb else -1, fmt)
+    d = support.load_dump(golden, "outputs")
     desc = cpu.desc_from_dump(d, out_format=fmt, stage_mask=abi.STAGE_SRGB if srgb else 0)
     got = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
-    assert got.dtype == want.dtype and got.shape == want.shape
-    assert np.array_equal(got.view(np.uint16) if got.dtype == np.float16 else got,
-                          want.view(np.uint16) if want.dtype == np.float16 else want)
-    fr.close()
+    assert got.shape == (*OUTPUT_FRAME[::-1], 4 if fmt == abi.OUT_RGBA_U8 else 3)
+    assert same(got, golden[f"outputs.{fmt}_{int(srgb)}"][0])
 
 
-@pytest.mark.parametrize("xs,ys", [(256, 256), (960, 540), (37, 21)])
-def test_dc_stage_bit_exact(xs, ys, refmod):
+@pytest.mark.parametrize("xs,ys", DC_CASES)
+def test_dc_stage_bit_exact(xs, ys, golden):
     """DequantDC + AdaptiveDCSmoothing of the reference (both builds) vs the restatement."""
     from oracle import cpu
     q = support.dc_stage_input(xs, ys)
     for variant in ("strict", "default"):
-        refmod.use_variant(variant)
-        try:
-            for mul in (1.0, 0.5):
-                assert np.array_equal(refmod.dequant_dc(q, support.DC_FACTORS, mul, support.DC_CFL),
-                                      cpu.dequant_dc(q, support.DC_FACTORS, mul, support.DC_CFL))
-            dc = cpu.dequant_dc(q, support.DC_FACTORS, 1.0, support.DC_CFL)
-            assert np.array_equal(refmod.adaptive_dc_smoothing(dc, support.DC_FACTORS, 3),
-                                  cpu.adaptive_dc_smoothing(dc, support.DC_FACTORS))
-        finally:
-            refmod.use_variant("strict")
+        want = golden[f"dc_{variant}_{xs}x{ys}"]
+        for k, mul in enumerate((1.0, 0.5)):
+            assert same(cpu.dequant_dc(q, support.DC_FACTORS, mul, support.DC_CFL), want[k]), (variant, mul)
+        dc = cpu.dequant_dc(q, support.DC_FACTORS, 1.0, support.DC_CFL)
+        assert same(cpu.adaptive_dc_smoothing(dc, support.DC_FACTORS), want[2]), variant
 
 
-@pytest.mark.parametrize("fmt,dtype,ch", [(abi.OUT_RGB_U8, np.uint8, 3), (abi.OUT_RGBA_U8, np.uint8, 4),
-                                          (abi.OUT_RGB_U16, np.uint16, 3), (abi.OUT_RGB_F16, np.float16, 3),
-                                          (abi.OUT_RGB_F32, np.float32, 3)])
-def test_full_chain_equals_default_public_decode(fmt, dtype, ch, refmod):
+@pytest.mark.parametrize("fmt,dtype,ch", PUBLIC_CASES)
+def test_full_chain_equals_default_public_decode(fmt, dtype, ch, golden, host_rcpss):
     """The path with JXLGPU_STAGE_SRGB and a packed output format is, byte for byte, what the reference's
     PUBLIC decoder delivers by default for an sRGB image (what `djxl in.jxl out.png` writes): public API
-    == hot path + FromLinear + WriteToOutput (reference stages) == the restatement (strict build)."""
+    == hot path + FromLinear + WriteToOutput (reference stages, checked when the golden data is made)
+    == the restatement (strict build)."""
     from oracle import cpu
-    img = wl.synth_image(333, 277, 5)
-    data = refmod.encode_rgb8(img, 1.0, 7, -1, -1, 2)
-    public = refmod.decode_native(data, (277, 333, ch), dtype, 2)
-    fr = refmod.Frame(data, 2)
-    d = fr.dump()
-    hot, _ = fr.render_out(-33, fmt)
-    fr.close()
+    img = wl.synth_image(*OUTPUT_FRAME, 5)
+    d = support.load_dump(golden, "outputs")
     desc = cpu.desc_from_dump(d, out_format=fmt, stage_mask=abi.STAGE_SRGB)
     restated = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
-
-    def bits(a):
-        return a.view(np.uint16) if a.dtype == np.float16 else a
-    assert np.array_equal(bits(public), bits(hot))
-    assert np.array_equal(bits(public), bits(restated))
+    assert restated.dtype == dtype and restated.shape == (*OUTPUT_FRAME[::-1], ch)
+    assert same(restated, golden[f"public.{fmt}"][0])
     # and it is a decode of the image that went in (8-bit sRGB in, d1.0): mean abs error < 2 %
     scale = {np.uint8: 255.0, np.uint16: 65535.0}.get(dtype, 1.0)
-    assert np.abs(public[..., :3].astype(np.float64) / scale - img / 255.0).mean() < 0.02
+    assert np.abs(restated[..., :3].astype(np.float64) / scale - img / 255.0).mean() < 0.02
 
 
 @pytest.mark.parametrize("distance", [1.0, 8.0])
@@ -217,57 +226,43 @@ def test_gpu_frame_binding_from_decoder_state(cfg, refmod):
     fr.close()
 
 
-@pytest.mark.parametrize("rs,w,h", [(2, 600, 300), (4, 1100, 210), (8, 2100, 160)])
-def test_upsampling_stage_bit_exact(rs, w, h, refmod):
+@pytest.mark.parametrize("rs,w,h", UPSAMPLING_CASES)
+def test_upsampling_stage_bit_exact(rs, w, h, golden, host_rcpss):
     """SURVEY.md §8f rank 4, UpsamplingStage (stage_upsampling.cc:51-271): frames encoded with resampling 2/4/8.
     The restatement (jxo_upsample_plane, after the filters and before XYB like PreparePipeline orders them) is
-    bit-exact against the reference's own stage, and the reference's hot path + stage equals its public decode."""
+    bit-exact against the reference's own stage, whose output is the reference's public decode (checked when
+    the golden data is made)."""
     from oracle import cpu
-    img = wl.synth_image(w, h, seed=rs)
-    data = refmod.encode_rgb8(img, 1.0, 7, -1, -1, 4, resampling=rs)
-    fr = refmod.Frame(data, 2)
-    i = fr.info
+    d = support.load_dump(golden, f"ups{rs}")
+    i = d.info
     assert i.upsampling == rs and (i.xsize_upsampled, i.ysize_upsampled) == (w, h)
-    d = fr.dump()
     desc = cpu.desc_from_dump(d)
     assert desc.upsampling == rs and desc.out_xsize == w and desc.out_ysize == h
     desc.out_format = abi.OUT_PLANAR_F32
-    chain = (1 if i.gab else 0) | (2 if i.epf_iters >= 3 else 0) | (4 if i.epf_iters >= 1 else 0) | (8 if i.epf_iters >= 2 else 0)
-    want, _ = fr.render(chain | refmod.STAGE_XYB | refmod.STAGE_UPSAMPLING)
-    assert want.shape == (3, h, w)
+    want, want_xyb = golden[f"ups{rs}.want"]
     got = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
-    assert np.array_equal(got, want)
-    desc.stage_mask = abi.STAGE_EXPLICIT | chain          # the upsampled XYB planes themselves
-    want_xyb, _ = fr.render(chain | refmod.STAGE_UPSAMPLING)
-    assert np.array_equal(cpu.render_frame(desc, d.coeffs, rcp_mode=1), want_xyb)
-    fr.close()
-    full = refmod.decode_linear_f32(data, 2)              # the decoder's real pipeline
-    assert np.array_equal(np.moveaxis(want, 0, 2), full)
+    assert got.shape == (3, h, w) and same(got, want)
+    desc.stage_mask = abi.STAGE_EXPLICIT | chain(i)          # the upsampled XYB planes themselves
+    assert same(cpu.render_frame(desc, d.coeffs, rcp_mode=1), want_xyb)
 
 
-@pytest.mark.parametrize("rs,w,h,iso", [(1, 600, 300, 3200), (2, 600, 299, 6400), (1, 523, 260, 1600)])
-def test_noise_stages_bit_exact(rs, w, h, iso, refmod):
+@pytest.mark.parametrize("rs,w,h,iso", NOISE_CASES)
+def test_noise_stages_bit_exact(rs, w, h, iso, golden, host_rcpss):
     """SURVEY.md §8f rank 4, noise: frames the reference encoder made with photon noise (frame flag kNoise).
     Random3Planes (dec_noise.cc:45-152) + ConvolveNoiseStage + AddNoiseStage (stage_noise.cc) restated in
-    oracle/jxl_oracle.c: bit-exact against the reference's own stages, alone and behind the upsampling, and the
-    reference's hot path + stages equals its public decode."""
+    oracle/jxl_oracle.c: bit-exact against the reference's own stages, alone and behind the upsampling, whose
+    output is the reference's public decode (checked when the golden data is made)."""
     from oracle import cpu
-    img = wl.synth_image(w, h, seed=rs + iso)
-    data = refmod.encode_rgb8(img, 1.0, 7, -1, -1, 4, resampling=rs | ((iso // 100) << 16))
-    fr = refmod.Frame(data, 2)
-    i = fr.info
+    d = support.load_dump(golden, f"noise{rs}_{w}x{h}_{iso}")
+    i = d.info
     assert i.noise == 1 and max(i.noise_lut) > 1e-3 and i.upsampling == rs
-    d = fr.dump()
     desc = cpu.desc_from_dump(d)
     assert desc.noise == 1 and (desc.visible_frame_index, desc.nonvisible_frame_index) == (1, 0)
     desc.out_format = abi.OUT_PLANAR_F32
-    chain = (1 if i.gab else 0) | (2 if i.epf_iters >= 3 else 0) | (4 if i.epf_iters >= 1 else 0) | (8 if i.epf_iters >= 2 else 0)
-    want, _ = fr.render(chain | refmod.STAGE_XYB | refmod.STAGE_UPSAMPLING | refmod.STAGE_NOISE)
-    assert np.array_equal(cpu.render_frame(desc, d.coeffs, rcp_mode=1), want)
-    without, _ = fr.render(chain | refmod.STAGE_XYB | refmod.STAGE_UPSAMPLING)
-    assert not np.array_equal(without, want)
-    fr.close()
-    assert np.array_equal(np.moveaxis(want, 0, 2), refmod.decode_linear_f32(data, 2))
+    got = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
+    assert same(got, golden[f"noise{rs}_{w}x{h}_{iso}.want"][0])
+    desc.noise = 0
+    assert not np.array_equal(cpu.render_frame(desc, d.coeffs, rcp_mode=1), got)
 
 
 def make_jpeg(w, h, quality, seed=5):
@@ -279,24 +274,21 @@ def make_jpeg(w, h, quality, seed=5):
     return b.getvalue()
 
 
-@pytest.mark.parametrize("w,h,q", [(600, 300, 90), (517, 331, 75)])
-def test_jpeg_origin_ycbcr_frames(w, h, q, refmod):
+@pytest.mark.parametrize("w,h,q", JPEG_CASES)
+def test_jpeg_origin_ycbcr_frames(w, h, q, golden, host_rcpss):
     """SURVEY.md §8f rank 4, YCbCr: a 4:4:4 JPEG recompressed by the reference encoder (JxlEncoderAddJPEGFrame) is a
     VarDCT frame with the YCbCr colour transform.  Dequantisation + IDCT are the XYB path's; the colour stage is
     kYCbCrStage (stage_ycbcr.cc:33-71).  Restatement bit-exact against the reference's stages, and its 8-bit output
     identical to the reference's PUBLIC decoder (no transfer function follows: the image is not XYB-encoded)."""
-    pytest.importorskip("PIL")
     from oracle import cpu
-    data = refmod.encode_jpeg(make_jpeg(w, h, q), 4)
-    fr = refmod.Frame(data, 2)
-    i = fr.info
+    d = support.load_dump(golden, f"jpeg{w}x{h}_{q}")
+    i = d.info
     assert i.ycbcr == 1 and i.gab == 0 and i.epf_iters == 0
-    d = fr.dump()
     desc = cpu.desc_from_dump(d)
     assert desc.color_transform == 1
+    want, public = golden[f"jpeg{w}x{h}_{q}.want"]
     desc.out_format = abi.OUT_PLANAR_F32
-    want, _ = fr.render(refmod.STAGE_XYB)          # bit 16 = the frame's colour transform
-    fr.close()
-    assert np.array_equal(cpu.render_frame(desc, d.coeffs, rcp_mode=1), want)
+    assert same(cpu.render_frame(desc, d.coeffs, rcp_mode=1), want)
     desc.out_format = abi.OUT_RGB_U8
-    assert np.array_equal(cpu.render_frame(desc, d.coeffs, rcp_mode=1), refmod.decode_native(data, (h, w, 3), np.uint8, 2))
+    got = cpu.render_frame(desc, d.coeffs, rcp_mode=1)
+    assert got.shape == (h, w, 3) and same(got, public)
